@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- Navier2D timesteps/s on B200 (BASELINE.json metric), one JSON line on stdout.
 
-  python bench.py --gpus N --steps K --warmup W [--config C2|C3|C4|C1] [--impl reference]
+  python bench.py --gpus N --steps K --warmup W [--config C2|C3|C4|C1] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one `Navier2D::update()` (src/navier_stokes/navier.rs:438-466) on synthetic fields:
 constructor defaults, physical fields U(-0.1, 0.1) from numpy default_rng(1/2/3), forward().
@@ -21,6 +21,8 @@ cpu_baseline / --impl reference: the C++/OpenMP restatement of the reference's u
 parity_check: 2 steps of a 257 x 129 problem on the same ranks against the numpy oracle (smooth state: 1e-10; white noise:
          max(1e-10, 10 x the oracle's own response to a last-bit change of its input)); parity_check_workload: the
          benchmarked configuration itself against the C++ restatement (1 GPU).
+--dump-outputs DIR: the four spectral state arrays (temp, velx, vely, pres) as the last timed step left them, written to
+         DIR/<name>.npy (see dump_outputs), so that two builds can be compared output for output on identical inputs.
 """
 import argparse
 import json
@@ -255,6 +257,28 @@ def time_ops(b2, ctx, cfg, eig, peak_gbs, world=1, calls=10, dist=None):
                     "27 lane passes of the step, so these do not add up to ms_per_step"}
 
 
+DUMP_BYTES = 64 * 10**6
+
+
+def dump_outputs(arrays, out_dir, budget=DUMP_BYTES):
+    """Write every array to out_dir/<name>.npy in float64 (complex arrays as [..., 2] = real, imaginary part), at most
+    `budget` bytes in all.  An array larger than its even share of the budget is replaced by a fixed sample of its flattened
+    entries, the same in every run: positions drawn without replacement by numpy default_rng(0), in ascending order."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    share = budget // len(arrays) - 4096   # room for the .npy header
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        cx = np.iscomplexobj(a)
+        width = 16 if cx else 8   # bytes per entry in the file
+        if a.size * width > share:
+            flat = a.reshape(-1)
+            a = flat[np.sort(np.random.default_rng(0).choice(flat.size, share // width, replace=False))]
+        out = np.stack([a.real, a.imag], axis=-1) if cx else a
+        np.save(os.path.join(out_dir, f"{name}.npy"), out.astype(np.float64, copy=False))
+
+
 def np_zeros_like_vhat(f):
     """a smooth, non-trivial spectral state for the standalone operator timings (timing is data-independent)"""
     import numpy as np
@@ -339,6 +363,8 @@ def main():
     ap.add_argument("--ops-multi", action="store_true", help="also time the standalone operators on N > 1 ranks (slab fields)")
     ap.add_argument("--no-parity", action="store_true", help="skip the in-run parity checks (small multi-rank problem; workload vs CPU restatement)")
     ap.add_argument("--mode", type=int, default=1, help="1 fused+graph (default), 3 fused without graph, 0 one pass pair per reference call")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the state arrays of the last timed step to DIR/<name>.npy (float64, at most 64 MB in all)")
     args = ap.parse_args()
     if args.config is None:
         # BASELINE.json quotes its metric "at 1/2/4/8 B200" on configs[3] = confined 4097 x 4097 (C4), which fits one GPU
@@ -400,6 +426,8 @@ def main():
     ms = ctx.timer_stop()
     fence()
     t_b = time.time()
+    # copied here: the clock, GEMM and e2e passes below step the same solver further
+    outputs = (nav.gather_state() if dist is not None else nav.state()) if args.dump_outputs else None
     if dist is not None:  # device time of the slowest rank
         t = torch.tensor([ms], dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -591,6 +619,8 @@ def main():
         "setup_s": setup_s, "div_norm": div,
     }
     if rank == 0:
+        if outputs is not None:
+            dump_outputs(outputs, args.dump_outputs)
         print(json.dumps(line), flush=True)
     if dist is not None:
         dist.barrier()
