@@ -72,6 +72,10 @@ int b2_space_destroy(b2_space* sp);
 /* shape_physical / shape_spectral / ortho shape; spectral & ortho of r2c spaces are complex */
 int b2_space_shape(const b2_space* sp, int shape_kind, int* rows, int* cols, int* is_complex);
 int b2_space_coords(const b2_space* sp, int axis, double* x_host /* n values */);
+/* diagnostic, no reference counterpart: the lane-kernel layout chosen for one pass orientation when the space was created
+ * (orient 0: lanes along axis 1, orient 1: lanes along axis 0).  out8 = {E points per thread, LN lanes per CTA, TPL threads
+ * per lane, fast (compile-time-geometry instance), CHW tiles per sub-chunk, sub-chunks per lane, threads per CTA, shared bytes} */
+int b2_space_lane_layout(const b2_space* sp, int orient, int* out8);
 
 /* ---- device arrays (the `Array2<T>` values that flow between Field and Solve calls) ---- */
 int b2_array_create(b2_space* sp, int shape_kind, b2_array** out);

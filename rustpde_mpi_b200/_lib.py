@@ -36,6 +36,7 @@ SYMBOLS = {
     "b2_space_destroy": (_I, [_P]),
     "b2_space_shape": (_I, [_P, _I, _IP, _IP, _IP]),
     "b2_space_coords": (_I, [_P, _I, _DP]),
+    "b2_space_lane_layout": (_I, [_P, _I, _IP]),
     "b2_array_create": (_I, [_P, _I, _PP]),
     "b2_array_destroy": (_I, [_P]),
     "b2_array_local_rows": (_I, [_P, _IP, _IP]),

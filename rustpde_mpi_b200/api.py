@@ -186,6 +186,15 @@ class Space2:
             out.append(x)
         return out
 
+    LAYOUT_KEYS = ("E", "LN", "TPL", "fast", "CHW", "nsc", "NT", "smem")
+
+    def lane_layout(self, orient):
+        """Diagnostic (no reference counterpart): the lane-kernel layout this space's passes run with, fixed when the space
+        was created.  orient 0: lanes along axis 1, orient 1: lanes along axis 0."""
+        out = (C.c_int * 8)()
+        check(lib().b2_space_lane_layout(self._h, orient, out))
+        return dict(zip(self.LAYOUT_KEYS, out))
+
 
 def _release(fn, handle):
     """Destroy a native object from close()/__del__: never raises (interpreter shutdown, already-destroyed context)."""

@@ -711,6 +711,9 @@ static int launch_pass(b2_ctx* ctx, const PassCfg& c, const LaneProg& p) {
   B2_INST(16, 2, 256) B2_INST(16, 2, 128)
   B2_INST(8, 4, 64) B2_INST(8, 4, 32) B2_INST(8, 4, 16) B2_INST(8, 4, 8) B2_INST(4, 4, 8) B2_INST(4, 4, 16) B2_INST(4, 4, 32)
 #undef B2_INST
+  // the launcher has already rewritten band ops into OP_BANDC / OP_PREBAND, which the generic instances do not implement:
+  // a fast layout that has_fast_instance accepts but the list above lacks would otherwise give wrong results without an error
+  if (c.fast) return fail(B2_ERR_ARG, "internal: fast layout E/LN/TPL without a compiled instance");
   if (c.LN == 4) {
     if (c.E == 16) return launch_ELT<16, 4, 0>(ctx, c, p);
     if (c.E == 8) return launch_ELT<8, 4, 0>(ctx, c, p);
@@ -1594,6 +1597,14 @@ int b2_space_coords(const b2_space* sp, int axis, double* x) {
   const Base1& b = sp->b[axis];
   const double PI = 3.14159265358979323846;
   for (int j = 0; j < b.n; j++) x[j] = b.cheb ? -std::cos(PI * j / (b.n - 1)) : 2.0 * PI * j / b.n;
+  return B2_OK;
+}
+int b2_space_lane_layout(const b2_space* sp, int orient, int* out8) {
+  if (!sp || !out8) return fail(B2_ERR_ARG, "b2_space_lane_layout: null");
+  if (orient < 0 || orient > 1) return fail(B2_ERR_ARG, "orient");
+  const PassCfg& c = sp->cfg[orient];
+  const int v[8] = {c.E, c.LN, c.TPL, c.fast ? 1 : 0, c.CHW, c.nsc, c.NT, (int)c.smem};
+  for (int i = 0; i < 8; i++) out8[i] = v[i];
   return B2_OK;
 }
 
